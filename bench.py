@@ -2,7 +2,7 @@
 """bench.py — headline benchmark of the hot path (BASELINE.json): agent requests/sec through
 ingest + dedupe + route on 512 B records.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c3|c2|c5]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload c3|c2|c5] [--dump-outputs DIR]
 
 A "step" is ONE pass of the hot path (K1: ingest + dedupe + route) over ONE batch of the workload's records.  The
 headline workload is c3 = BASELINE configs[2], the largest single-GPU configuration and the one with duplicate
@@ -19,6 +19,9 @@ c2 = configs[1] (1 M records, uniform, no duplicates) and both id modes are repo
             itself cannot be built in this image) timed on ONE host core over a bounded sample.
   --impl reference  times that CPU restatement on all host threads (agents sharded across threads) on the same
             workload/metric — the reference arm the driver compares against.
+  --dump-outputs DIR  after the timed steps, the verdicts of the last one as DIR/verdict_<field>.npy (float64).  The
+            records are seeded and the key of the minted ids is fixed, so the same arguments give the same inputs in every
+            run and two builds can be compared output for output.
 Under torchrun (N > 1) every rank owns one GPU and one shard of the agents; no data-path collective is needed
 for c2/c3 (records are steered to the owner shard before the copy), so scaling is "weak".
 """
@@ -34,9 +37,11 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the bench runs from a built tree that may be read-only: it leaves no __pycache__ there
 
 METRIC = "agent_requests_per_sec_ingest_dedupe_route_512B"
 ALG_BYTES_PER_RECORD = 520          # SURVEY.md 8(d): 512 B record read + 4 B queue/state entry + 4 B verdict
+ID_SECRET = 0x9E3779B97F4A7C15      # key of the engine-minted ids of the headline run (AGR_CFG_MINT_IDS)
 WORKLOADS = {
     "c2": dict(name="C2: 1M synthetic 512B POST /agent/<id>/chat records per step, 256 agent ids, uniform, all agents running, no crash-replay",
                records=1 << 20, agents=256, zipf_milli=0, dup_permille=0),
@@ -431,7 +436,7 @@ def run_c4(args, rank, world, local_rank):
         dist.init_process_group("gloo", rank=0, world_size=1)
     local_cpus = bind_to_gpu_numa_node(local_rank)
     B, W = 1 << 20, args.warmup
-    S = args.steps if args.steps != 200 else 10                  # 10 x 1 M = 10 M records per GPU unless --steps says otherwise
+    S = args.steps if args.steps is not None else 10             # 10 x 1 M = 10 M records per GPU unless --steps says otherwise
     e_steps, e_warm = min(S, args.e2e_steps), 1
     rows = int((W + S + e_warm + e_steps + 1) * B * 1.1)
     eng = A.Engine(device=local_rank, slab_rows=rows, max_agents=1024, max_batch=B, k1_variant=args.variant,
@@ -515,6 +520,21 @@ def run_c4(args, rank, world, local_rank):
     dist.destroy_process_group()
 
 
+def dump_verdicts(out_dir, route):
+    """--dump-outputs: the verdicts of one timed step as agr_ingest_rows would hand them to its caller (agr_verdict
+    {code, flags, http_status, agent_slot}).  The timed launches leave them on the device as one route word per row
+    (slot in bits 0..22, code in 23..25, AGR_VF_* flags from bit 26); the fields are unpacked here the way k1_verdict_word
+    does on the device, one float64 array per field (4 x 8 MiB for a 1 M-record step)."""
+    from agentainer_lab_b200 import constants as K
+    route = route.astype(np.int64)
+    code = (route >> 23) & 0x7
+    http = np.select([code == K.AGR_V_QUEUED, code == K.AGR_V_UNAVAILABLE, code == K.AGR_V_NOT_FOUND], [202, 503, 404], 0)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("verdict_code", code), ("verdict_flags", route >> 26), ("verdict_http_status", http),
+                    ("verdict_agent_slot", route & 0x7FFFFF)):
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64))
+
+
 def run_ours(args, wl, rank, world, local_rank):
     import torch
     import agentainer_lab_b200 as A
@@ -532,8 +552,9 @@ def run_ours(args, wl, rank, world, local_rank):
     e_steps, e_warm = min(S, args.e2e_steps), 1
     rows = max(args.rows, (W + S) * B + (e_warm + e_steps) * B + (B if world > 1 else 0) * 2)
     id_flags = K.AGR_CFG_MINT_IDS if args.id_mode == "mint" else 0
+    # a fixed id key: the minted ids, and with them the records that name them and the verdicts, are the same in every run
     eng = A.Engine(device=local_rank, slab_rows=rows, max_agents=1024, max_batch=B, k1_variant=args.variant | (args.timing_stride << 16),
-                   flags=K.AGR_CFG_PERSISTENCE | K.AGR_CFG_TIMING | args.diag_flags | id_flags)
+                   flags=K.AGR_CFG_PERSISTENCE | K.AGR_CFG_TIMING | args.diag_flags | id_flags, id_secret=ID_SECRET)
     nanos0 = 1700000000000000000 + rank * 10_000_000_000        # each rank (shard) owns its own agent ids
     for k in range(wl["agents"]):
         eng.set_agent_state(A.synth_agent_id(k, agent_nanos0=nanos0), "running")
@@ -571,6 +592,8 @@ def run_ours(args, wl, rank, world, local_rank):
     clocks = sampler.stop()
     st = eng.stats()
     assert st["ingested"] == (W + S) * B, st
+    if args.dump_outputs and rank == 0:
+        dump_verdicts(args.dump_outputs, eng.debug_read("route", first + (W + S - 1) * B, B))
     if args.diag_flags:
         print("WARNING: diagnostic flags set; numbers below are for attribution only", file=sys.stderr)
     # ---- e2e through the public C-ABI call with pinned host buffers (H2D + kernels + D2H verdicts timed)
@@ -798,7 +821,7 @@ def run_c5(args, rank, world, local_rank):
     torch.cuda.set_device(local_rank)
     n, na, W = 1 << 18, 256, max(3, args.warmup)
     total_target = 100_000_000 if world == 8 else 6_000_000 * world
-    S = args.steps if args.steps != 200 else -(-total_target // (world * n))
+    S = args.steps if args.steps is not None else -(-total_target // (world * n))
     R = 8 * n
     TTLB = 4                                                           # a record lives four batches
     rng = np.random.default_rng(7 + rank)
@@ -929,7 +952,7 @@ def run_c5(args, rank, world, local_rank):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=None, help="timed steps (default 200; c4: 10; c5: enough batches for its record target)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="c3", choices=sorted(WORKLOADS) + ["c4", "c5"])
@@ -945,7 +968,14 @@ def main():
     ap.add_argument("--x-steps", type=int, default=3)
     ap.add_argument("--diag-flags", type=lambda x: int(x, 0), default=0, help="extra AGR_CFG_DIAG_* bits (results invalid; attribution only)")
     ap.add_argument("--rows", type=int, default=0, help="override slab rows (table size follows)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="c2 / c3: write the verdicts of the last timed step to DIR/verdict_<field>.npy (float64)")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.workload not in WORKLOADS):
+        ap.error("--dump-outputs covers the GPU path of the c2 / c3 workloads")
+    if args.steps is None and (args.impl == "reference" or args.workload in WORKLOADS):
+        args.steps = 200
     args.warmup = max(3, args.warmup) if args.impl == "ours" else args.warmup
     rank, world = int(os.environ.get("RANK", 0)), int(os.environ.get("WORLD_SIZE", 1))
     local_rank = int(os.environ.get("LOCAL_RANK", 0))

@@ -50,6 +50,44 @@ def test_gojson_string_property():
 import pytest
 
 
+def test_bench_arguments_are_checked():
+    """--steps sets the number of timed steps (at least one); --dump-outputs covers the GPU path of c2 / c3 only.  Both are
+    refused before any work starts, so this runs without a GPU."""
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "out"], ["--workload", "c5", "--dump-outputs", "out"]):
+        res = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *extra], capture_output=True, text=True, timeout=120, cwd=ROOT)
+        assert res.returncode == 2 and "error:" in res.stderr and res.stdout == "", (extra, res.stderr)
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_the_same_in_every_run(tmp_path):
+    """--dump-outputs writes the verdicts of the last timed step, and two runs with the same arguments write the same
+    arrays (seeded records, fixed key of the minted ids)."""
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    from agentainer_lab_b200 import constants as K
+    runs = []
+    for k in range(2):
+        out = tmp_path / f"run{k}"
+        res = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "3", "--no-other-mode", "--no-callers",
+                              "--no-secondary", "--no-cpu", "--e2e-steps", "1", "--dump-outputs", str(out)],
+                             capture_output=True, text=True, timeout=900, cwd=ROOT)
+        assert res.returncode == 0, res.stderr[-2000:]
+        assert json.loads([l for l in res.stdout.splitlines() if l.startswith("{")][0])["steps"] == 2
+        runs.append({p.name: np.load(p) for p in out.iterdir()})
+    a, b = runs
+    assert sorted(a) == ["verdict_agent_slot.npy", "verdict_code.npy", "verdict_flags.npy", "verdict_http_status.npy"]
+    assert sum(x.nbytes for x in a.values()) <= 64 << 20
+    for name, x in a.items():
+        assert x.dtype == np.float64 and x.shape == (1 << 20,) and np.array_equal(x, b[name]), name
+    # C3: every agent is running, so every request is forwarded; ~10 % are replay-flagged, every other one is stored and tracked
+    assert (a["verdict_code.npy"] == K.AGR_V_FORWARD).all() and (a["verdict_http_status.npy"] == 0).all()
+    flags = a["verdict_flags.npy"].astype(np.int64)
+    replay = (flags & K.AGR_VF_REPLAY) != 0
+    assert 0.05 < replay.mean() < 0.15
+    assert ((flags[~replay] & (K.AGR_VF_STORED | K.AGR_VF_TRACKED)) == (K.AGR_VF_STORED | K.AGR_VF_TRACKED)).all()
+    assert len(np.unique(a["verdict_agent_slot.npy"])) <= 256
+
+
 @pytest.mark.gpu
 def test_gpu_arm_line():
     res = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "4", "--warmup", "3", "--no-other-mode", "--no-callers", "--e2e-steps", "2"],
