@@ -62,6 +62,11 @@ class AgrSynth(C.Structure):
                 ("mint_base_rid", C.c_uint64), ("mint_secret", C.c_uint64), ("mint_shard", C.c_uint32), ("mint_gen", C.c_uint32)]
 
 
+class AgrResult(C.Structure):
+    """agr_result: what agr_poll / agr_wait hand back for a ticket"""
+    _fields_ = [("verdict", C.c_uint8 * 8), ("request_id", C.c_uint8 * 16), ("rid", C.c_uint64), ("result", C.c_int32), ("is_outcome", C.c_uint32)]
+
+
 # every symbol include/agentainer_gpu.h declares (tests/test_abi.py cross-checks this list against the header)
 ABI_SYMBOLS = [
     "agr_create", "agr_destroy", "agr_abi_version", "agr_last_error", "agr_strerror",
@@ -72,6 +77,7 @@ ABI_SYMBOLS = [
     "agr_agent_hash", "agr_agent_shard", "agr_comm_unique_id", "agr_comm_init", "agr_ingest_sharded", "agr_complete_sharded", "agr_snapshot", "agr_restore", "agr_verify", "agr_store_response_body", "agr_get_response_body",
     "agr_store_response", "agr_store_error_text", "agr_get_record_json", "agr_pending_json", "agr_rows_json", "agr_expire", "agr_reclaim", "agr_set_agent_states", "agr_json_decode",
     "agr_submit_ingest", "agr_submit_complete", "agr_poll", "agr_wait", "agr_ring_capacity", "agr_ingest_sharded_rows", "agr_fill_rows", "agr_reclaim_async",
+    "agr_submit_ingest_var",
 ]
 
 _lib = None
@@ -156,6 +162,9 @@ def load_library(path: Optional[str] = None) -> C.CDLL:
         "agr_complete_sharded": (i32, [vp, vp, u32, vp, C.POINTER(AgrExchangeInfo)]),
         "agr_ingest_sharded_rows": (i32, [vp, u64, u32, vp, C.POINTER(AgrExchangeInfo)]),
         "agr_fill_rows": (i32, [vp, u64, vp, u32]),
+        "agr_submit_ingest_var": (i32, [vp, vp, u32, C.POINTER(u64)]),
+        "agr_poll": (i32, [vp, u64, C.POINTER(AgrResult)]),
+        "agr_wait": (i32, [vp, u64, C.POINTER(AgrResult)]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)
@@ -395,6 +404,25 @@ class Engine:
         first = C.c_uint64()
         _check(self.lib, self.lib.agr_ingest_var(self.h, _ptr(blob), _ptr(offsets), n, _ptr(out), _ptr(ids), C.byref(first)))
         return out, ids, first.value
+
+    def submit_ingest_var(self, rec: np.ndarray) -> Optional[int]:
+        """agr_submit_ingest_var: ONE record in the agr_ingest_var wire form; the ticket, or None on AGR_EAGAIN (collect, then again)."""
+        assert rec.dtype == np.uint8 and rec.flags["C_CONTIGUOUS"]
+        t = C.c_uint64()
+        rc = self.lib.agr_submit_ingest_var(self.h, _ptr(rec), len(rec), C.byref(t))
+        if rc == K.AGR_EAGAIN:
+            return None
+        _check(self.lib, rc)
+        return t.value
+
+    def poll(self, ticket: int, wait: bool = False):
+        """agr_poll (agr_wait with wait=True): (verdict, request id, row, result) of a record's ticket, or None while undecided."""
+        r = AgrResult()
+        rc = (self.lib.agr_wait if wait else self.lib.agr_poll)(self.h, ticket, C.byref(r))
+        if rc == K.AGR_EAGAIN:
+            return None
+        _check(self.lib, rc)
+        return np.frombuffer(bytes(r.verdict), dtype=verdict_dtype)[0], bytes(r.request_id), r.rid, r.result
 
     def replay_scan_var(self, cap: int = 1 << 14, blob_cap: int = 1 << 24):
         while True:

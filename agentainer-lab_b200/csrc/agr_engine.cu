@@ -276,14 +276,16 @@ static void pack_agent_id(const char* id, unsigned long long w[4]) {
 // Host side of agr_svc.h.  Lock-free for the callers: one fetch_add claims ring slots, the payload is written into pinned
 // device-mapped memory, a release store publishes it, and the caller waits on a word the GPU writes.  One dispatcher thread
 // per handle turns the published prefix of the ring into batch descriptors; the resident service kernel (k_svc) does the rest.
-extern "C" { static int reserve_rows_locked(agr_handle* h, uint32_t n, uint64_t* first); }
-cudaError_t agr_launch_svc(const agr_dev& d, const svc_dev& v, const agr_k2_scratch& k2, unsigned long long next_seq, cudaStream_t st);
+extern "C" { static int reserve_rows_locked(agr_handle* h, uint32_t n, uint64_t* first);
+             static int reserve_var_locked(agr_handle* h, uint32_t n, uint64_t bytes, uint64_t* first, uint64_t* base); }
+cudaError_t agr_launch_svc(const agr_dev& d, const svc_dev& v, const agr_k2_scratch& k2, unsigned long long next_seq, bool var, cudaStream_t st);
 unsigned long long agr_svc_desc_check(const svc_desc* dsc);
 
 struct svc_host {
     // ---- read-mostly (every caller reads these on every call; nothing here is written while callers run)
     svc_desc* desc = nullptr; uint8_t* payload = nullptr; svc_res* res = nullptr; svc_ctl* ctl = nullptr;   // pinned, device-mapped
     std::atomic<uint32_t>* ready = nullptr;             // [SVC_SLOTS] (lap + 1) << 2 | SVC_OP_* once the slot's payload is complete
+    uint32_t* lens = nullptr;                           // [SVC_SLOTS] pinned, device-mapped: stored length of a run's record (AGR_CFG_VARLEN)
     uint32_t spin_cpus = 1;                             // how many waiters may spin (CPU allowance minus dispatcher and driver threads)
     std::atomic<bool> shutdown{false}, sleeping{false}; // (sleeping flips only when the ring has been empty for 2 ms)
     std::atomic<int> fatal{0};                          // a CUDA error in the dispatcher: every later call fails with it
@@ -337,14 +339,14 @@ static int svc_start_locked(agr_handle* h) {
     svc_host* s = h->svc;
     if (s->running) return 0;
     svc_dev v{};
-    v.desc = s->desc; v.payload = s->payload; v.res = s->res; v.ctl = s->ctl; v.dupfix = s->d_dupfix;
+    v.desc = s->desc; v.payload = s->payload; v.lens = s->lens; v.res = s->res; v.ctl = s->ctl; v.dupfix = s->d_dupfix;
     v.idle_ns = 2000000000ULL;                                   // safety only: the dispatcher stops the kernel long before
     s->ctl->state = 1; s->ctl->stop = 0;
     std::atomic_thread_fence(std::memory_order_seq_cst);
     sync_window(h);
     // resume at the first batch the previous incarnation did not run (normally none is pending; a batch published right
     // before this launch is)
-    cudaError_t e = agr_launch_svc(h->d, v, s->k2, s->ctl->done_seq + 1, h->stream);
+    cudaError_t e = agr_launch_svc(h->d, v, s->k2, s->ctl->done_seq + 1, (h->cfg.flags & AGR_CFG_VARLEN) != 0, h->stream);
     if (e != cudaSuccess) { s->fatal = AGR_ECUDA; return fail(AGR_ECUDA, std::string("service kernel launch: ") + cudaGetErrorString(e)); }
     s->running = true;
     s->starts++;
@@ -365,12 +367,13 @@ struct HLock {
     HLock(const HLock&) = delete; HLock& operator=(const HLock&) = delete;
 };
 
-// answers every op of [from, to) from the host side (slab full, CUDA error): the callers see rc
+// answers every op of [from, to) from the host side (slab full, CUDA error): the callers see rc.  Backwards, so that the
+// continuation cells of a run get their tag before its head's answer (its collector then releases every cell of the run).
 static void svc_fail_ops(svc_host* s, uint64_t from, uint64_t to, int rc, bool records_only) {
-    for (uint64_t a = from; a < to; ++a) {
+    for (uint64_t a = to; a-- > from;) {
         const uint32_t slot = (uint32_t)(a & (SVC_SLOTS - 1u));
         const uint32_t rw = s->ready[slot].load(std::memory_order_relaxed), kd = rw & 3u;
-        const bool rec = kd == SVC_OP_RECORD;
+        const bool rec = kd == SVC_OP_RECORD || kd == SVC_OP_CONT;
         // (a skipped slot has no waiter and keeps its old answer; it may even have been published again for the NEXT lap already)
         if ((rw >> 2) != (uint32_t)(a / SVC_SLOTS) + 1u || kd == SVC_OP_SKIP || (records_only && !rec)) continue;
         svc_res* r = s->res + slot;
@@ -390,8 +393,14 @@ static void svc_dispatcher(agr_handle* h) {
     uint64_t to = s->taken;
     uint32_t nrec = 0;
     uint32_t kinds[SVC_MAX_OPS / 16] = {0};
+    // variable-length records: runs of slots, 128 record slots per batch (one shared-memory stage of k_svc), and their bytes
+    const bool var = (h->cfg.flags & AGR_CFG_VARLEN) != 0;
+    uint32_t nslots = 0;
+    uint64_t nbytes = 0;
     while (!s->shutdown.load(std::memory_order_acquire)) {
-        svc_scan(s, s->taken, &to, &nrec, kinds, 128u);           // (csrc/agr_ring.hpp: shared with the CPU simulation of the ring)
+        // (csrc/agr_ring.hpp: shared with the CPU simulations of the ring)
+        if (var) svc_scan_run(s, s->taken, &to, &nrec, &nslots, &nbytes, kinds, 128u);
+        else svc_scan(s, s->taken, &to, &nrec, kinds, 128u);
         const auto now = std::chrono::steady_clock::now();
         if (to == s->taken) {
             const auto idle = std::chrono::duration_cast<std::chrono::microseconds>(now - last_work).count();
@@ -422,28 +431,30 @@ static void svc_dispatcher(agr_handle* h) {
         }
         spins = 0;
         std::lock_guard<std::mutex> hl(h->mu);
-        if (s->fatal.load()) { svc_fail_ops(s, s->taken, to, s->fatal.load(), false); s->taken = to; nrec = 0; memset(kinds, 0, sizeof kinds); continue; }
+        if (s->fatal.load()) { svc_fail_ops(s, s->taken, to, s->fatal.load(), false); s->taken = to; nrec = 0; nslots = 0; nbytes = 0; memset(kinds, 0, sizeof kinds); continue; }
         if (s->running && s->ctl->state != 1u) {                // it left on its own (safety timeout): note it and start another
             cudaStreamSynchronize(h->stream);
             s->running = false;
         }
         // a resident kernel blocks device-wide synchronisations of other threads (cudaFree ...): let it go every 20 ms
         if (s->running && std::chrono::duration_cast<std::chrono::milliseconds>(now - s->started).count() > 20) svc_stop_locked(h);
-        uint64_t first = 0;
+        uint64_t first = 0, vbase = 0;
         bool have_rows = true;
         if (nrec) {
-            if (reserve_rows_locked(h, nrec, &first) < 0) { svc_fail_ops(s, s->taken, to, AGR_ENOSPC, true); have_rows = false; }
+            const int rc = var ? reserve_var_locked(h, nrec, nbytes, &first, &vbase) : reserve_rows_locked(h, nrec, &first);
+            if (rc < 0) { svc_fail_ops(s, s->taken, to, var ? rc : AGR_ENOSPC, true); have_rows = false; }
         }
         svc_desc dsc{};
         for (uint32_t k = 0; k < (uint32_t)(to - s->taken); ++k) {
             uint32_t kd = (kinds[k >> 4] >> ((k & 15u) * 2u)) & 3u;
-            if (kd == SVC_OP_RECORD && !have_rows) kd = SVC_OP_SKIP;
+            if ((kd == SVC_OP_RECORD || kd == SVC_OP_CONT) && !have_rows) kd = SVC_OP_SKIP;
             dsc.kinds[k >> 4] |= kd << ((k & 15u) * 2u);
         }
         dsc.from = s->taken; dsc.count = (uint32_t)(to - s->taken); dsc.n_records = have_rows ? nrec : 0u;
         dsc.first_l = first; dsc.first_p = (uint32_t)phys_row(h, first);
         dsc.tail = h->tail; dsc.head_l = h->rows_used; dsc.tail_phys = is_ring(h) ? (uint32_t)(h->tail % h->cfg.slab_rows) : 0u;
         dsc.idx_base = h->d.idx_base;
+        dsc.vbase = vbase;
         dsc.seq = s->seq + 1;
         dsc.check = agr_svc_desc_check(&dsc);
         svc_desc* slot = s->desc + (dsc.seq % SVC_DESCS);
@@ -457,10 +468,11 @@ static void svc_dispatcher(agr_handle* h) {
         s->seq = dsc.seq;
         s->taken = to;
         s->batches.fetch_add(1, std::memory_order_relaxed);
-        s->ops.fetch_add(dsc.count, std::memory_order_relaxed);
+        const uint32_t nops = dsc.count - (var ? nslots - nrec : 0u);   // operations (a run is one)
+        s->ops.fetch_add(nops, std::memory_order_relaxed);
         h->k1_launches += nrec ? 1 : 0;                         // accounting: batches with records / with outcomes served by k_svc
-        h->k2_launches += (dsc.count > nrec) ? 1 : 0;
-        nrec = 0; memset(kinds, 0, sizeof kinds);
+        h->k2_launches += (nops > nrec) ? 1 : 0;
+        nrec = 0; nslots = 0; nbytes = 0; memset(kinds, 0, sizeof kinds);
         if (!s->running && svc_start_locked(h) < 0) {
             // could not launch: nothing will ever process this batch — fail it from here
             svc_fail_ops(s, dsc.from, to, AGR_ECUDA, false);
@@ -498,6 +510,7 @@ static int svc_create(agr_handle* h) {
     TRY(pin((void**)&s->desc, sizeof(svc_desc) * SVC_DESCS));
     TRY(pin((void**)&s->payload, (size_t)SVC_SLOTS * SVC_PAYLOAD));
     TRY(pin((void**)&s->res, sizeof(svc_res) * SVC_SLOTS));
+    TRY(pin((void**)&s->lens, sizeof(uint32_t) * SVC_SLOTS));
     TRY(pin((void**)&s->ctl, sizeof(svc_ctl)));
     s->ready = new std::atomic<uint32_t>[SVC_SLOTS];
     for (uint32_t i = 0; i < SVC_SLOTS; ++i) s->ready[i].store(0);
@@ -576,6 +589,27 @@ static int svc_complete(agr_handle* h, const agr_outcome* outs, uint32_t n, int3
         svc_release(s, pos[i]);
     }
     if (rc < 0) return fail(rc, "single-request front end: CUDA error");
+    return 0;
+}
+// variable-length records (offsets already checked): one run of slots per record, in call order
+static int svc_ingest_var(agr_handle* h, const uint8_t* blob, const uint32_t* offsets, uint32_t n, agr_verdict* out, uint8_t (*ids)[16],
+                          uint64_t* first_rid) {
+    svc_host* s = h->svc;
+    uint64_t pos[SVC_MAX_CALL];
+    for (uint32_t i = 0; i < n; ++i)
+        while (!svc_submit_run(s, blob + offsets[i], offsets[i + 1] - offsets[i], &pos[i])) {}    // a run not free: draw again
+    int rc = 0;
+    for (uint32_t i = 0; i < n; ++i) {
+        svc_answer r; svc_wait(s, pos[i], &r);
+        if ((r.w0 & 0xffu) == 0u) rc = (int)r.w1;
+        else {
+            if (out) { memcpy(&out[i], &r.w0, 4); memcpy((uint8_t*)&out[i] + 4, &r.w1, 4); }
+            if (ids) svc_request_id(h, pos[i], r.rid, ids[i]);
+            if (i == 0 && first_rid) *first_rid = r.rid;
+        }
+        svc_release_run(s, pos[i], svc_run_slots(offsets[i + 1] - offsets[i]));
+    }
+    if (rc < 0) return fail(rc, rc == AGR_ENOSPC ? "byte slab or slab full" : rc == AGR_EINVAL ? "batch larger than half the byte slab" : "single-request front end: CUDA error");
     return 0;
 }
 
@@ -731,7 +765,7 @@ static int create_impl(const agr_config* cfg_in, agr_handle* h) {
     TRY(dev_alloc(h, &h->d_goff, (size_t)c.max_agents + 2, false));
     TRY(dev_alloc(h, &h->d_min_inq, (size_t)1, false));
     CK(cudaStreamSynchronize(h->stream));
-    if ((c.flags & AGR_CFG_COMBINE) && !varlen) TRY(svc_create(h));
+    if (c.flags & AGR_CFG_COMBINE) TRY(svc_create(h));
     return 0;
 }
 
@@ -1082,7 +1116,9 @@ static int ingest_ex_locked(agr_handle* h, const agr_record* recs, uint32_t n, a
 
 // ------------------------------------------------------------------------------------------ tickets (submit / collect)
 uint32_t agr_ring_capacity(void) { return SVC_SLOTS; }
-#define TICKET_OUTCOME (1ULL << 63)                               // a ticket = ring slot number | kind
+#define TICKET_OUTCOME (1ULL << 63)                               // a ticket = ring slot number | kind | (run length - 1) << 59
+#define TICKET_RUN_SHIFT 59
+#define TICKET_SLOT ((1ULL << TICKET_RUN_SHIFT) - 1ULL)
 static int submit_one(agr_handle* h, uint32_t kind, const void* item, size_t bytes, agr_ticket* ticket) {
     if (!h || !item || !ticket) return fail(AGR_EINVAL, "NULL argument");
     svc_host* s = h->svc;
@@ -1092,12 +1128,27 @@ static int submit_one(agr_handle* h, uint32_t kind, const void* item, size_t byt
     *ticket = a | (kind == SVC_OP_OUTCOME ? TICKET_OUTCOME : 0ULL);
     return 0;
 }
-int agr_submit_ingest(agr_handle* h, const agr_record* rec, agr_ticket* ticket) { return submit_one(h, SVC_OP_RECORD, rec, sizeof(agr_record), ticket); }
+int agr_submit_ingest(agr_handle* h, const agr_record* rec, agr_ticket* ticket) {
+    if (h && (h->cfg.flags & AGR_CFG_VARLEN)) return fail(AGR_EINVAL, "variable-length engine: use agr_submit_ingest_var");
+    return submit_one(h, SVC_OP_RECORD, rec, sizeof(agr_record), ticket);
+}
+static bool var_len_ok(uint32_t len) { return !(len & 15u) && len >= AGR_HEADER_BYTES && len <= AGR_VAR_MAX_RECORD; }
+int agr_submit_ingest_var(agr_handle* h, const uint8_t* rec, uint32_t len, agr_ticket* ticket) {
+    if (!h || !rec || !ticket) return fail(AGR_EINVAL, "NULL argument");
+    if (!(h->cfg.flags & AGR_CFG_VARLEN)) return fail(AGR_EINVAL, "engine was not created with AGR_CFG_VARLEN");
+    svc_host* s = h->svc;
+    if (!s) return fail(AGR_EINVAL, "engine was not created with AGR_CFG_COMBINE");
+    if (!var_len_ok(len)) return fail(AGR_EINVAL, "record length must be a multiple of 16 in [96, 8192]");
+    uint64_t a = 0;
+    if (!svc_submit_run(s, rec, len, &a)) return AGR_EAGAIN;            // collect outstanding tickets (agr_poll) and come again
+    *ticket = a | (uint64_t)(svc_run_slots(len) - 1u) << TICKET_RUN_SHIFT;
+    return 0;
+}
 int agr_submit_complete(agr_handle* h, const agr_outcome* outcome, agr_ticket* ticket) { return submit_one(h, SVC_OP_OUTCOME, outcome, sizeof(agr_outcome), ticket); }
 static int collect(agr_handle* h, agr_ticket ticket, const svc_answer& r, agr_result* out) {
     svc_host* s = h->svc;
     const bool rec = !(ticket & TICKET_OUTCOME);
-    const uint64_t t = ticket & ~TICKET_OUTCOME;
+    const uint64_t t = ticket & TICKET_SLOT;
     if (out) {
         memset(out, 0, sizeof *out);
         out->is_outcome = rec ? 0u : 1u;
@@ -1106,19 +1157,19 @@ static int collect(agr_handle* h, agr_ticket ticket, const svc_answer& r, agr_re
             else { memcpy(&out->verdict, &r.w0, 4); memcpy((uint8_t*)&out->verdict + 4, &r.w1, 4); out->rid = r.rid; svc_request_id(h, t, r.rid, out->request_id); }
         } else out->result = (int32_t)r.w0;
     }
-    svc_release(s, t);
+    svc_release_run(s, t, (uint32_t)((ticket >> TICKET_RUN_SHIFT) & 15u) + 1u);
     return 0;
 }
 int agr_poll(agr_handle* h, agr_ticket ticket, agr_result* out) {
     if (!h || !h->svc) return fail(AGR_EINVAL, "engine was not created with AGR_CFG_COMBINE");
     svc_answer r;
-    if (!svc_try(h->svc, ticket & ~TICKET_OUTCOME, &r)) return AGR_EAGAIN;
+    if (!svc_try(h->svc, ticket & TICKET_SLOT, &r)) return AGR_EAGAIN;
     return collect(h, ticket, r, out);
 }
 int agr_wait(agr_handle* h, agr_ticket ticket, agr_result* out) {
     if (!h || !h->svc) return fail(AGR_EINVAL, "engine was not created with AGR_CFG_COMBINE");
     svc_answer r;
-    svc_wait(h->svc, ticket & ~TICKET_OUTCOME, &r);
+    svc_wait(h->svc, ticket & TICKET_SLOT, &r);
     return collect(h, ticket, r, out);
 }
 
@@ -1344,36 +1395,47 @@ int agr_get_record(agr_handle* h, const char* agent_id, const uint8_t request_id
 }
 
 // ------------------------------------------------------------------------------------------ variable-length records
+// rows and byte-slab space for n records of `bytes` stored bytes in all (agr_ingest_var, and the dispatcher of the single-request
+// front end for a batch): *base = physical byte offset of the first.  Byte ring: the records never wrap either.  Nothing is
+// reserved unless both fit.
+static int reserve_var_locked(agr_handle* h, uint32_t n, uint64_t bytes, uint64_t* first, uint64_t* base) {
+    uint64_t vpad = 0;
+    if (!is_ring(h)) {
+        if (h->vused + bytes > h->vcap) return fail(AGR_ENOSPC, "byte slab full");
+    } else {
+        if (bytes > h->vcap / 2) return fail(AGR_EINVAL, "batch larger than half the byte slab");
+        const uint64_t at = h->vused % h->vcap;
+        vpad = (at + bytes > h->vcap) ? h->vcap - at : 0;
+        if (h->vused + vpad + bytes - h->vtail > h->vcap) return fail(AGR_ENOSPC, "byte slab full: agr_expire + agr_reclaim release bytes at the tail");
+    }
+    TRY(reserve_rows_locked(h, n, first));
+    h->vused += vpad;
+    *base = is_ring(h) ? h->vused % h->vcap : h->vused;
+    h->vused += bytes;
+    return 0;
+}
 int agr_ingest_var(agr_handle* h, const uint8_t* blob, const uint32_t* offsets, uint32_t n, agr_verdict* out, uint8_t (*ids)[16],
                    uint64_t* first_rid) {
     if (!h || (n && (!blob || !offsets))) return fail(AGR_EINVAL, "NULL argument");
     if (!(h->cfg.flags & AGR_CFG_VARLEN)) return fail(AGR_EINVAL, "engine was not created with AGR_CFG_VARLEN");
+    auto shape_ok = [&]() -> int {
+        if (offsets[0] != 0) return fail(AGR_EINVAL, "offsets[0] must be 0");
+        for (uint32_t i = 0; i < n; ++i)                          // host-side shape check (lengths are part of the wire format)
+            if (offsets[i + 1] < offsets[i] || !var_len_ok(offsets[i + 1] - offsets[i]))
+                return fail(AGR_EINVAL, "record " + std::to_string(i) + ": length must be a multiple of 16 in [96, 8192]");
+        return 0;
+    };
+    if (h->svc && n >= 1 && n <= SVC_MAX_CALL) { TRY(shape_ok()); return svc_ingest_var(h, blob, offsets, n, out, ids, first_rid); }
     HLock lk(h);
     CK(cudaSetDevice(h->device));
     if (n > h->cfg.max_batch) return fail(AGR_EINVAL, "n exceeds max_batch");
     uint64_t first = 0;
     if (n == 0) { if (first_rid) *first_rid = h->rows_used; return 0; }
     const uint64_t bytes = offsets[n];
-    if (offsets[0] != 0) return fail(AGR_EINVAL, "offsets[0] must be 0");
-    for (uint32_t i = 0; i < n; ++i) {                           // host-side shape check (lengths are part of the wire format)
-        const uint32_t len = offsets[i + 1] - offsets[i];
-        if (offsets[i + 1] < offsets[i] || (len & 15u) || len < AGR_HEADER_BYTES || len > AGR_VAR_MAX_RECORD)
-            return fail(AGR_EINVAL, "record " + std::to_string(i) + ": length must be a multiple of 16 in [96, 8192]");
-    }
-    uint64_t vpad = 0;
-    if (!is_ring(h)) {
-        if (h->vused + bytes > h->vcap) return fail(AGR_ENOSPC, "byte slab full");
-    } else {                                                      // byte ring: a blob never wraps either
-        if (bytes > h->vcap / 2) return fail(AGR_EINVAL, "batch larger than half the byte slab");
-        const uint64_t at = h->vused % h->vcap;
-        vpad = (at + bytes > h->vcap) ? h->vcap - at : 0;
-        if (h->vused + vpad + bytes - h->vtail > h->vcap) return fail(AGR_ENOSPC, "byte slab full: agr_expire + agr_reclaim release bytes at the tail");
-    }
-    TRY(reserve_rows_locked(h, n, &first));
+    TRY(shape_ok());
+    uint64_t base = 0;
+    TRY(reserve_var_locked(h, n, bytes, &first, &base));
     if (first_rid) *first_rid = first;
-    h->vused += vpad;
-    const uint64_t base = is_ring(h) ? h->vused % h->vcap : h->vused;          // physical byte offset of the blob
-    h->vused += bytes;
     cudaStream_t st = h->stream;
     CK(cudaMemcpyAsync(h->d.slab + base, blob, bytes, cudaMemcpyHostToDevice, st));
     if (is_pinned(offsets)) CK(cudaMemcpyAsync(h->d_voffsets, offsets, ((size_t)n + 1) * 4, cudaMemcpyHostToDevice, st));

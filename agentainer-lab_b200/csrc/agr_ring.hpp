@@ -5,6 +5,7 @@
 //   svc_res* res; uint8_t* payload; std::atomic<uint32_t>* ready;          pinned, device-mapped in the engine
 //   std::atomic<uint64_t> head, scanned; std::atomic<uint32_t> waiters; uint32_t spin_cpus;
 //   std::atomic<bool> sleeping; std::mutex smu; std::condition_variable scv;   the dispatcher's sleep / wake-up
+//   uint32_t* lens;                                                        runs only (svc_submit_run, svc_scan_run): pinned, device-mapped
 // The dispatcher (engine) or its stand-in (simulation) consumes ready words in slot order, keeps `scanned` = first slot whose
 // ready word it has not consumed, and sees to it that every consumed operation other than SVC_OP_SKIP gets its 16-byte answer.
 #pragma once
@@ -78,6 +79,52 @@ static bool svc_submit_one(H* s, uint32_t kind, const void* item, size_t item_by
     *abs = a;
     return ok;
 }
+
+// ---- runs (AGR_CFG_VARLEN): a record of stored length len takes svc_run_slots(len) consecutive slots, possibly across the ring's
+// end.  Every slot of the run obeys the slot-reuse rule above, the GPU answers every cell of it (the continuation cells with
+// their tag only, before the head's answer) and the collector releases every cell, so svc_slot_free needs nothing new.
+static inline uint32_t svc_run_slots(uint32_t len) { return (len + SVC_PAYLOAD - 1u) / SVC_PAYLOAD; }
+// hands ONE variable-length record over.  true: *abs is its head slot (ticket); false: some slot of the run was not free, and
+// the whole run has been published as no-ops.
+template <class H>
+static bool svc_submit_run(H* s, const uint8_t* rec, uint32_t len, uint64_t* abs) {
+    const uint32_t k = svc_run_slots(len);
+    const uint64_t a = s->head.fetch_add(k, std::memory_order_relaxed);
+    bool ok = true;
+    for (uint32_t j = 0; j < k && ok; ++j) {
+        const uint64_t b = a + j;
+        ok = svc_slot_free(s, b, (uint32_t)(b & (SVC_SLOTS - 1u)), (uint32_t)(b / SVC_SLOTS));
+    }
+    if (ok) {
+        for (uint32_t j = 0; j < k; ++j) {                       // slot by slot: the run may cross the ring's end
+            __m128i* dst = reinterpret_cast<__m128i*>(s->payload + (size_t)((a + j) & (SVC_SLOTS - 1u)) * SVC_PAYLOAD);
+            const __m128i* src = reinterpret_cast<const __m128i*>(rec + (size_t)j * SVC_PAYLOAD);
+            const uint32_t n = (j + 1u == k ? len - j * SVC_PAYLOAD : SVC_PAYLOAD) / 16u;
+            for (uint32_t c = 0; c < n; ++c) _mm_stream_si128(dst + c, _mm_loadu_si128(src + c));
+        }
+        _mm_sfence();
+        __atomic_store_n(&s->lens[a & (SVC_SLOTS - 1u)], len, __ATOMIC_RELAXED);
+        for (uint32_t j = 1; j < k; ++j) {
+            const uint64_t b = a + j;
+            s->ready[b & (SVC_SLOTS - 1u)].store(((uint32_t)(b / SVC_SLOTS) + 1u) << 2 | SVC_OP_CONT, std::memory_order_relaxed);
+        }
+        // the head last: a scanner that sees it published sees the length word and the whole run
+        s->ready[a & (SVC_SLOTS - 1u)].store(((uint32_t)(a / SVC_SLOTS) + 1u) << 2 | SVC_OP_RECORD, std::memory_order_release);
+    } else {
+        // a slot's ready word may be overwritten only once the dispatcher has consumed the previous lap's (the slots after the one
+        // that failed were not looked at)
+        uint32_t w = 0;
+        while (s->scanned.load(std::memory_order_acquire) + SVC_SLOTS <= a + k - 1u) cpu_relax(w);
+        for (uint32_t j = 0; j < k; ++j) {
+            const uint64_t b = a + j;
+            s->ready[b & (SVC_SLOTS - 1u)].store(((uint32_t)(b / SVC_SLOTS) + 1u) << 2 | SVC_OP_SKIP, std::memory_order_release);
+        }
+    }
+    if (s->sleeping.load(std::memory_order_seq_cst)) { std::lock_guard<std::mutex> lk(s->smu); s->scv.notify_one(); }
+    *abs = a;
+    return ok;
+}
+
 struct svc_answer { uint32_t w0, w1; uint64_t rid; };
 template <class H>
 static inline bool svc_try(H* s, uint64_t a, svc_answer* out) {
@@ -109,6 +156,10 @@ template <class H>
 static inline void svc_release(H* s, uint64_t a) {       // everything of the answer (and of the payload) has been read
     __atomic_store_n(&s->res[a & (SVC_SLOTS - 1u)].w[3], (svc_tag(a) | SVC_COLLECTED) << 16, __ATOMIC_RELEASE);
 }
+template <class H>
+static inline void svc_release_run(H* s, uint64_t a, uint32_t k) {      // every cell of a run (k slots from a)
+    for (uint32_t j = 0; j < k; ++j) svc_release(s, a + j);
+}
 
 // ---- the dispatcher's side of the ready words
 // Grows the contiguous published prefix [taken, *to) by whatever has been published since: at most SVC_MAX_OPS operations and
@@ -125,6 +176,32 @@ static inline void svc_scan(H* s, const uint64_t taken, uint64_t* to, uint32_t* 
         if ((rw & 3u) == SVC_OP_RECORD) { if (*nrec == max_records) break; (*nrec)++; }
         kinds[(*to - taken) >> 4] |= (rw & 3u) << (((*to - taken) & 15u) * 2u);
         (*to)++;
+    }
+    if (*to != s->scanned.load(std::memory_order_relaxed)) s->scanned.store(*to, std::memory_order_release);
+}
+// svc_scan for rings that carry runs: the budget is max_slots RECORD SLOTS (a run of k slots counts k) and a run is taken whole or
+// left for the next batch (an empty batch takes any run: k <= 16).  Continuation slots are noted as SVC_OP_CONT without reading
+// their ready words (the head's release store covers them).  *nslots / *nbytes: record slots / stored bytes taken so far.
+template <class H>
+static inline void svc_scan_run(H* s, const uint64_t taken, uint64_t* to, uint32_t* nrec, uint32_t* nslots, uint64_t* nbytes,
+                                uint32_t* kinds, const uint32_t max_slots) {
+    while (*to - taken < SVC_MAX_OPS) {
+        const uint32_t slot = (uint32_t)(*to & (SVC_SLOTS - 1u));
+        const uint32_t rw = s->ready[slot].load(std::memory_order_acquire);
+        if ((rw >> 2) != (uint32_t)(*to / SVC_SLOTS) + 1u) break;
+        const uint32_t kd = rw & 3u;
+        uint32_t k = 1;
+        if (kd == SVC_OP_RECORD) {
+            const uint32_t len = __atomic_load_n(&s->lens[slot], __ATOMIC_RELAXED);
+            k = svc_run_slots(len);
+            if (*nslots + k > max_slots || *to - taken + k > SVC_MAX_OPS) break;
+            (*nrec)++; *nslots += k; *nbytes += len;
+        }
+        for (uint32_t j = 0; j < k; ++j) {
+            const uint64_t p = *to + j - taken;
+            kinds[p >> 4] |= (j ? (uint32_t)SVC_OP_CONT : kd) << ((p & 15u) * 2u);
+        }
+        *to += k;
     }
     if (*to != s->scanned.load(std::memory_order_relaxed)) s->scanned.store(*to, std::memory_order_release);
 }

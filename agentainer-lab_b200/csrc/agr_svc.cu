@@ -10,6 +10,9 @@
 //             (a block scan instead of k2_append's decoupled look-back: the whole batch is in this CTA);
 // then writes verdict, Request.ID, row and result code of every operation back to host memory, fences, and flips the
 // per-slot done words the callers spin on.  Integer / byte work only; nothing here is on a tensor core.
+// Two instantiations: fixed-stride 512 B records (one slot each), and variable-length records (AGR_CFG_VARLEN: a record's run of
+// k = ceil(len / 512) slots lands in k consecutive stage slots and goes to the byte slab at the batch's base + the sum of the
+// stored lengths before it, as k1_ingest_var would put it).
 #include "agr_device.cuh"
 #include "agr_svc.h"
 
@@ -23,6 +26,14 @@
 #define SVC_MAX_RECS 128u                                   // records per batch that fit one shared-memory stage
 #define SVC_STAGE (SVC_MAX_RECS * 512u + SVC_MAX_OPS * 64u) // 80 KiB
 #define SVC_SMEM (2u * SVC_STAGE)                           // 160 KiB
+// variable-length records: behind each stage, per record its stored length, its byte offset in the batch and its first stage
+// slot, then the batch's record-slot count and the loader warps' partial sums (a maximal 8192 B record is 16 of the 128 slots)
+#define SVC_VX_LEN 0u
+#define SVC_VX_VOFF (SVC_MAX_RECS * 4u)
+#define SVC_VX_FIRST (SVC_MAX_RECS * 8u)
+#define SVC_VX_MISC (SVC_MAX_RECS * 10u)
+#define SVC_STAGE_VAR (SVC_STAGE + SVC_MAX_RECS * 10u + 32u)   // 81.3 KiB
+#define SVC_SMEM_VAR (2u * SVC_STAGE_VAR)                   // 162.6 KiB
 #define BAR_FULL0 1
 #define BAR_FREE0 3
 #define BAR_WORK 5
@@ -51,8 +62,10 @@ __host__ __device__ __forceinline__ unsigned long long svc_mix_word(uint32_t w, 
     return ((unsigned long long)w + 0x9e3779b97f4a7c15ULL * (i + 1u)) * (0xbf58476d1ce4e5b9ULL + 2ULL * i);
 }
 
-extern "C" __global__ void __launch_bounds__(SVC_THREADS, 1)
+template <bool VAR>
+__global__ void __launch_bounds__(SVC_THREADS, 1)
 k_svc(const agr_dev d0, const svc_dev v, const agr_k2_scratch k2, const unsigned long long first_seq) {
+    constexpr uint32_t STAGE = VAR ? SVC_STAGE_VAR : SVC_STAGE;
     extern __shared__ __align__(128) uint8_t smem[];
     __shared__ __align__(16) uint32_t s_dw[2][64];           // the accepted descriptors, as words
     __shared__ uint32_t s_go[2], s_nout[2];
@@ -69,8 +82,13 @@ k_svc(const agr_dev d0, const svc_dev v, const agr_k2_scratch k2, const unsigned
         for (unsigned long long seq = first_seq;; ++seq) {
             const uint32_t st = (uint32_t)(seq & 1ULL);
             if (seq >= first_seq + 2ULL) bar_sync(BAR_FREE0 + (int)st, SVC_THREADS);      // the workers are done with batch seq - 2
-            uint8_t* s_rec = smem + st * SVC_STAGE;
+            uint8_t* s_rec = smem + st * STAGE;
             uint8_t* s_out = s_rec + SVC_MAX_RECS * 512u;
+            uint8_t* s_vx = s_rec + SVC_STAGE;                                  // (VAR only)
+            uint32_t* vx_len = reinterpret_cast<uint32_t*>(s_vx + SVC_VX_LEN);
+            uint32_t* vx_voff = reinterpret_cast<uint32_t*>(s_vx + SVC_VX_VOFF);
+            uint16_t* vx_first = reinterpret_cast<uint16_t*>(s_vx + SVC_VX_FIRST);
+            uint32_t* vx_misc = reinterpret_cast<uint32_t*>(s_vx + SVC_VX_MISC);   // [0] record slots, [4..7] loader warp sums
             if (warp == 0) {
                 const svc_desc* dp = v.desc + (seq % SVC_DESCS);
                 uint32_t go = 2u;                                               // 2 = keep polling
@@ -105,19 +123,29 @@ k_svc(const agr_dev d0, const svc_dev v, const agr_k2_scratch k2, const unsigned
                 __syncwarp();
                 uint32_t nout = 0;
                 if (go == 1u) {
-                    // op -> (record i | outcome j) maps: thirty-two ops per step, running offsets
+                    // op -> (record i | outcome j) maps: thirty-two ops per step, running offsets.  Variable-length records:
+                    // s_rec_op maps STAGE SLOTS (record and continuation slots in ring order) to ops, vx_first record -> slot
                     const svc_desc& D = *reinterpret_cast<const svc_desc*>(s_dw[st]);
-                    uint32_t br = 0, bo = 0;
+                    uint32_t br = 0, bo = 0, bs = 0;
                     const uint32_t lt = (1u << lane) - 1u;
                     for (uint32_t base = 0; base < D.count; base += 32u) {
                         const uint32_t op = base + lane;
                         const uint32_t kind = (op < D.count) ? ((D.kinds[op >> 4] >> ((op & 15u) * 2u)) & 3u) : 0u;
                         const uint32_t mr = __ballot_sync(FULL, kind == SVC_OP_RECORD), mo = __ballot_sync(FULL, kind == SVC_OP_OUTCOME);
-                        if (kind == SVC_OP_RECORD) s_rec_op[st][br + __popc(mr & lt)] = (uint16_t)op;
+                        if constexpr (VAR) {
+                            const bool in_run = kind == SVC_OP_RECORD || kind == SVC_OP_CONT;
+                            const uint32_t ms = __ballot_sync(FULL, in_run), js = bs + __popc(ms & lt);
+                            if (in_run) s_rec_op[st][js] = (uint16_t)op;
+                            if (kind == SVC_OP_RECORD) vx_first[br + __popc(mr & lt)] = (uint16_t)js;
+                            bs += __popc(ms);
+                        } else {
+                            if (kind == SVC_OP_RECORD) s_rec_op[st][br + __popc(mr & lt)] = (uint16_t)op;
+                        }
                         if (kind == SVC_OP_OUTCOME) s_out_op[st][bo + __popc(mo & lt)] = (uint16_t)op;
                         br += __popc(mr); bo += __popc(mo);
                     }
                     nout = bo;
+                    if constexpr (VAR) { if (lane == 0) vx_misc[0] = bs; }
                     last_work = globaltimer_ns();
                 }
                 if (lane == 0) {
@@ -131,8 +159,12 @@ k_svc(const agr_dev d0, const svc_dev v, const agr_k2_scratch k2, const unsigned
             if (go == 1u) {
                 // pull the payloads out of host memory: eight 16-byte loads in flight per thread
                 const svc_desc& D = *reinterpret_cast<const svc_desc*>(s_dw[st]);
-                const uint32_t rec_chunks = D.n_records * 32u, total = rec_chunks + s_nout[st] * 4u;
+                const uint32_t rec_chunks = (VAR ? vx_misc[0] : D.n_records) * 32u, total = rec_chunks + s_nout[st] * 4u;
                 const unsigned long long from = D.from;
+                uint32_t len = 0;                                               // (VAR) record tid's length word: same round trip
+                if constexpr (VAR) {
+                    if (tid < D.n_records) len = ld_sys_u32(v.lens + ((from + s_rec_op[st][vx_first[tid]]) & (SVC_SLOTS - 1u)));
+                }
                 for (uint32_t cb = tid; cb < total; cb += SVC_LOADERS * 8u) {
                     uint4 val[8];
 #pragma unroll
@@ -154,6 +186,16 @@ k_svc(const agr_dev d0, const svc_dev v, const agr_k2_scratch k2, const unsigned
                             *reinterpret_cast<uint4*>(dst) = val[u];
                         }
                     }
+                }
+                if constexpr (VAR) {                                            // byte offsets: exclusive scan of the lengths
+                    uint32_t x = len;
+#pragma unroll
+                    for (int o = 1; o < 32; o <<= 1) { const uint32_t y = __shfl_up_sync(FULL, x, o); if ((int)lane >= o) x += y; }
+                    if (lane == 31u) vx_misc[4 + warp] = x;
+                    bar_sync(BAR_LOAD, SVC_LOADERS);
+                    uint32_t pre = 0;
+                    for (uint32_t w = 0; w < warp; ++w) pre += vx_misc[4 + w];
+                    if (tid < D.n_records) { vx_len[tid] = len; vx_voff[tid] = pre + x - len; }
                 }
                 if (tid == 0) { const long long c = clock64(); c_load += c - c0; c0 = c; s_cyc[0] = c_wait; s_cyc[1] = c_load; }
             }
@@ -178,8 +220,11 @@ k_svc(const agr_dev d0, const svc_dev v, const agr_k2_scratch k2, const unsigned
             return;
         }
         const long long cw0 = clock64();
-        const uint8_t* s_rec = smem + st * SVC_STAGE;
+        const uint8_t* s_rec = smem + st * STAGE;
         const uint8_t* s_out = s_rec + SVC_MAX_RECS * 512u;
+        const uint32_t* vx_len = reinterpret_cast<const uint32_t*>(s_rec + SVC_STAGE + SVC_VX_LEN);     // (VAR only)
+        const uint32_t* vx_voff = reinterpret_cast<const uint32_t*>(s_rec + SVC_STAGE + SVC_VX_VOFF);
+        const uint16_t* vx_first = reinterpret_cast<const uint16_t*>(s_rec + SVC_STAGE + SVC_VX_FIRST);
         const svc_desc& D = *reinterpret_cast<const svc_desc*>(s_dw[st]);
         const uint32_t nrec = D.n_records, nout = s_nout[st];
         const unsigned long long from = D.from;
@@ -188,29 +233,60 @@ k_svc(const agr_dev d0, const svc_dev v, const agr_k2_scratch k2, const unsigned
         const uint32_t lt = (1u << lane) - 1u;
 
         // ------------------------------------------------------------------ records: slab rows + checksum (warp per record)
-        for (uint32_t i = wwarp; i < nrec; i += SVC_WORKERS / 32u) {
-            const uint32_t rid = D.first_p + i;
-            const uint4 x = lds_v4(s_rec + (size_t)i * 512u + lane * 16u);
-            *reinterpret_cast<uint4*>(d.slab + (size_t)rid * AGR_REC + lane * 16u) = x;
-            uint32_t c0 = x.x + x.y + x.z + x.w;
-            uint32_t c1 = (4u * lane + 1u) * x.x + (4u * lane + 2u) * x.y + (4u * lane + 3u) * x.z + (4u * lane + 4u) * x.w;
-            c0 = __reduce_add_sync(FULL, c0); c1 = __reduce_add_sync(FULL, c1);
-            if (lane == 0) d.cksum[rid] = agr_cksum_pack(c0, c1);
+        if constexpr (VAR) {
+            // lane = 16 B chunk, looping over records longer than 512 B; then the continuation cells' tags, fenced before the
+            // head's answer (which goes out after the barrier below): the collector sets SVC_COLLECTED in every cell of the run
+            // once it has seen the head's, and a late tag store would take it away again
+            for (uint32_t i = wwarp; i < nrec; i += SVC_WORKERS / 32u) {
+                const uint32_t rid = D.first_p + i, len = vx_len[i], j0 = vx_first[i];
+                const uint8_t* src = s_rec + (size_t)j0 * 512u;
+                uint8_t* dst = d.slab + D.vbase + vx_voff[i];
+                uint32_t c0 = 0, c1 = 0;
+                for (uint32_t c = lane; c < (len >> 4); c += 32u) {
+                    const uint4 x = lds_v4(src + (size_t)c * 16u);
+                    *reinterpret_cast<uint4*>(dst + (size_t)c * 16u) = x;
+                    c0 += x.x + x.y + x.z + x.w;
+                    c1 += (4u * c + 1u) * x.x + (4u * c + 2u) * x.y + (4u * c + 3u) * x.z + (4u * c + 4u) * x.w;
+                }
+                c0 = __reduce_add_sync(FULL, c0); c1 = __reduce_add_sync(FULL, c1);
+                if (lane == 0) d.cksum[rid] = agr_cksum_pack(c0, c1);
+                const uint32_t k = (len + SVC_PAYLOAD - 1u) / SVC_PAYLOAD;
+                if (k > 1u) {                                                    // warp-uniform
+                    if (lane >= 1u && lane < k) {
+                        const unsigned long long slot_abs = from + s_rec_op[st][j0 + lane];
+                        st_res(v.res + (slot_abs & (SVC_SLOTS - 1u)), 0u, 0u, 0u, svc_tag(slot_abs) << 16);
+                    }
+                    __threadfence_system();
+                }
+            }
+        } else {
+            for (uint32_t i = wwarp; i < nrec; i += SVC_WORKERS / 32u) {
+                const uint32_t rid = D.first_p + i;
+                const uint4 x = lds_v4(s_rec + (size_t)i * 512u + lane * 16u);
+                *reinterpret_cast<uint4*>(d.slab + (size_t)rid * AGR_REC + lane * 16u) = x;
+                uint32_t c0 = x.x + x.y + x.z + x.w;
+                uint32_t c1 = (4u * lane + 1u) * x.x + (4u * lane + 2u) * x.y + (4u * lane + 3u) * x.z + (4u * lane + 4u) * x.w;
+                c0 = __reduce_add_sync(FULL, c0); c1 = __reduce_add_sync(FULL, c1);
+                if (lane == 0) d.cksum[rid] = agr_cksum_pack(c0, c1);
+            }
         }
         // ------------------------------------------------------------------ records: decision chain, one record per thread
         uint32_t lc[K1_NLC + 1];
 #pragma unroll
         for (int c = 0; c <= K1_NLC; ++c) lc[c] = 0;
         if (wt < nrec) {
-            const uint8_t* hp = s_rec + (size_t)wt * 512u;
+            const uint8_t* hp = s_rec + (size_t)(VAR ? vx_first[wt] : wt) * 512u;
             const uint4 h0 = lds_v4(hp), h1 = lds_v4(hp + 16), h2 = lds_v4(hp + 32), h3 = lds_v4(hp + 48), h4 = lds_v4(hp + 64), h5 = lds_v4(hp + 80);
             const uint32_t rid = D.first_p + wt;
             k1_ctx cx;
-            k1_begin(d, k1_agent_issue(d, h2, h3), h0, h1, h2, h3, h4, h5.x, AGR_REC - AGR_OFF_PAYLOAD, 0ULL, cx);
+            k1_begin(d, k1_agent_issue(d, h2, h3), h0, h1, h2, h3, h4, h5.x, (VAR ? vx_len[wt] : AGR_REC) - AGR_OFF_PAYLOAD, 0ULL, cx);
             const k1_result r = k1_finish(d, rid, h1, h5, cx, lc);
             d.state[rid] = r.state;
             d.route[rid] = r.route;
-            if ((r.state & ST_STORED) && (d.cfg_flags & AGR_CFG_RING)) {         // TTL bookkeeping (see k1_note_time)
+            if constexpr (VAR) {                                                  // the row words k1_ingest_var leaves (its TTL
+                d.voff[rid] = D.vbase + vx_voff[wt];                              // bounds are agr_expire's: k1v_note_time)
+                d.vlen[rid] = vx_len[wt];
+            } else if ((r.state & ST_STORED) && (d.cfg_flags & AGR_CFG_RING)) {   // TTL bookkeeping (see k1_note_time)
                 unsigned long long t = pack64(h4.x, h4.y);
                 atomicMin(d.cmin + rid / AGR_CHUNK_ROWS, t ? t : 1ULL);
                 d.mtime[rid] = t;
@@ -224,7 +300,7 @@ k_svc(const agr_dev d0, const svc_dev v, const agr_k2_scratch k2, const unsigned
             if (wt < nrec) {
                 const uint32_t rid = D.first_p + wt;
                 const uint32_t r = k1_post_one(d, rid, dupfix, delta);
-                const unsigned long long slot_abs = from + s_rec_op[st][wt], lrow = D.first_l + wt;
+                const unsigned long long slot_abs = from + s_rec_op[st][VAR ? vx_first[wt] : wt], lrow = D.first_l + wt;
                 const uint2 vw = k1_verdict_word(r);
                 st_res(v.res + (slot_abs & (SVC_SLOTS - 1u)), vw.x, vw.y, (uint32_t)lrow, (uint32_t)((lrow >> 32) & 0xffffu) | (svc_tag(slot_abs) << 16));
             }
@@ -295,14 +371,16 @@ k_svc(const agr_dev d0, const svc_dev v, const agr_k2_scratch k2, const unsigned
     }
 }
 
-cudaError_t agr_launch_svc(const agr_dev& d, const svc_dev& v, const agr_k2_scratch& k2, unsigned long long next_seq, cudaStream_t st) {
-    static bool attr_done = false;
-    if (!attr_done) {
-        cudaError_t e = cudaFuncSetAttribute(k_svc, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SVC_SMEM);
+cudaError_t agr_launch_svc(const agr_dev& d, const svc_dev& v, const agr_k2_scratch& k2, unsigned long long next_seq, bool var, cudaStream_t st) {
+    static bool attr_done[2] = {false, false};
+    const uint32_t smem = var ? SVC_SMEM_VAR : SVC_SMEM;
+    if (!attr_done[var]) {
+        cudaError_t e = cudaFuncSetAttribute(var ? k_svc<true> : k_svc<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return e;
-        attr_done = true;
+        attr_done[var] = true;
     }
-    k_svc<<<1, SVC_THREADS, SVC_SMEM, st>>>(d, v, k2, next_seq);
+    if (var) k_svc<true><<<1, SVC_THREADS, smem, st>>>(d, v, k2, next_seq);
+    else k_svc<false><<<1, SVC_THREADS, smem, st>>>(d, v, k2, next_seq);
     return cudaGetLastError();
 }
 

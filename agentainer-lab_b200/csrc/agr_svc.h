@@ -5,9 +5,12 @@
 // the call pattern at the boundary is "many OS threads, ONE request per call": agr_ingest_ex(n = 1) then agr_complete(n = 1).
 // A kernel launch per call would cap the engine near 10^5 requests/s.  Instead:
 //   callers     claim ring slots with one fetch_add, write their record / outcome into PINNED, device-mapped host memory,
-//               publish the slot, and spin (then yield) on the slot's result word;
-//   dispatcher  one thread per handle: takes the contiguous published prefix of the ring (<= SVC_MAX_OPS), reserves slab rows
-//               for its records under the handle mutex and publishes a 256 B batch descriptor;
+//               publish the slot, and spin (then yield) on the slot's result word;  a variable-length record (AGR_CFG_VARLEN)
+//               takes a RUN of ceil(len / 512) consecutive slots: continuation slots (SVC_OP_CONT) are published first, the
+//               head slot (SVC_OP_RECORD) last, and its stored length goes into the per-slot length word before that;
+//   dispatcher  one thread per handle: takes the contiguous published prefix of the ring (<= SVC_MAX_OPS, <= 128 record slots,
+//               a run whole or not at all), reserves slab rows (and, AGR_CFG_VARLEN, slab bytes) for its records under the handle
+//               mutex and publishes a 256 B batch descriptor;
 //   service kernel  ONE resident CTA polls the descriptor ring over PCIe, pulls the batch's payloads straight out of host
 //               memory, runs the K1 decision chain (records) and the K2 state machine (outcomes) of agr_device.cuh on them,
 //               and writes verdict / id / row / result back into host memory.  No launch, no cudaMemcpy and no stream
@@ -19,12 +22,13 @@
 #include <stdint.h>
 
 #define SVC_SLOTS 16384u          // ring slots (power of two)
-#define SVC_MAX_OPS 256u          // operations per batch (<= 128 of them records: what one shared-memory stage of the kernel holds)
+#define SVC_MAX_OPS 256u          // ring slots per batch (<= 128 of them record slots: what one shared-memory stage of the kernel holds)
 #define SVC_MAX_CALL 32u          // records / outcomes per call that go through the ring
 #define SVC_DESCS 64u             // descriptor ring entries
 #define SVC_PAYLOAD 512u          // bytes per slot: an agr_record, or an agr_outcome in the first 64 B
 
-enum { SVC_OP_SKIP = 0, SVC_OP_RECORD = 1, SVC_OP_OUTCOME = 2 };
+// SVC_OP_CONT: slot 2 .. k of a variable-length record's run (its head slot is the SVC_OP_RECORD right before them)
+enum { SVC_OP_SKIP = 0, SVC_OP_RECORD = 1, SVC_OP_OUTCOME = 2, SVC_OP_CONT = 3 };
 
 // batch descriptor (256 B = 64 words), written by the dispatcher (host), polled by the kernel: sixteen lanes read 16 B each
 // in ONE poll; the kernel accepts it when the batch number matches and the check word agrees with the other 62 words (a poll
@@ -39,7 +43,9 @@ struct __attribute__((aligned(64))) svc_desc {
     uint32_t tail_phys;                   // live window of the slab after this batch's rows were reserved
     uint64_t tail, head_l;
     uint64_t idx_base;
-    uint64_t reserved[15];
+    uint64_t vbase;                       // AGR_CFG_VARLEN: physical slab byte offset of the first record (the others follow it in
+                                          // ring order, each at the sum of the stored lengths before it)
+    uint64_t reserved[14];
     uint64_t check;                       // words 60..61: XOR of svc_mix_word over words 0..59 and 62..63
     uint64_t seq;                         // words 62..63: batch number; the kernel waits for desc[seq % SVC_DESCS].seq == seq
 };
@@ -53,6 +59,8 @@ static_assert(sizeof(svc_desc) == 256, "svc_desc must be 256 B (sixteen 16 B lan
 //   outcome  w0 = (uint32_t)result (0 / AGR_ENOTFOUND / error code)
 //   w3 >> 16 = tag of the slot's lap (svc_tag): the caller spins on it, and sets SVC_COLLECTED in it once it has read the
 //              answer — that line is in the collector's cache anyway, so freeing a slot costs no extra miss.
+//   continuation slot of a run: only the tag; it is written BEFORE the head's answer (so the collector's SVC_COLLECTED, which
+//              it sets in every cell of the run, can never be overwritten by it)
 // Request.ID is not shipped: with engine-minted ids it is a function of the row (agr_mint_id, computed by the caller's
 // thread), with caller-supplied ids the caller has it already.
 struct __attribute__((aligned(16))) svc_res { volatile uint32_t w[4]; };
@@ -77,6 +85,7 @@ static_assert(sizeof(svc_res) == 16, "svc_res must be 16 B");
 struct svc_dev {                          // device-visible addresses of the pinned ring (UVA: host pointer == device pointer)
     const svc_desc* desc;
     const uint8_t* payload;               // [SVC_SLOTS][SVC_PAYLOAD]
+    const uint32_t* lens;                 // [SVC_SLOTS] AGR_CFG_VARLEN: stored length of the record whose run starts at the slot
     svc_res* res;                         // [SVC_SLOTS]
     svc_ctl* ctl;
     uint32_t* dupfix;                     // device word for in-batch duplicate ids (hash-id mode)

@@ -101,7 +101,9 @@ typedef struct agr_record {
                                        published, and ONE resident service kernel decides the batch and writes verdicts / ids / result
                                        codes straight back into host memory — no launch, copy or stream sync per request.  Event
                                        order: batch by batch; inside a batch records in ring order, then outcomes in ring order (all
-                                       of them were in flight together).  Fixed-stride engines only (ignored with AGR_CFG_VARLEN). */
+                                       of them were in flight together).  With AGR_CFG_VARLEN the same holds for agr_ingest_var and
+                                       agr_complete with n <= 32 (a record of stored length L takes ceil(L / 512) consecutive ring
+                                       slots) and agr_submit_ingest_var; results are those of the batch calls. */
 #define AGR_CFG_RING          0x40u /* the slab is a ring (with AGR_CFG_VARLEN the byte slab is a ring too): row ids keep counting arrivals, a
                                        record lives at row id mod slab_rows, and agr_reclaim hands the rows at the tail that no longer hold
                                        a record (agr_expire) back for reuse — a shard then runs indefinitely instead of filling up.
@@ -239,6 +241,12 @@ typedef struct agr_result {
 } agr_result;                  /* 40 B */
 int agr_submit_ingest(agr_handle* h, const agr_record* rec, agr_ticket* ticket);
 int agr_submit_complete(agr_handle* h, const agr_outcome* outcome, agr_ticket* ticket);
+/* AGR_CFG_VARLEN | AGR_CFG_COMBINE: agr_submit_ingest for ONE variable-length record in the agr_ingest_var wire form (96 B header,
+ * payload zero padded to 16 B; len = its stored length, a multiple of 16 in [96, AGR_VAR_MAX_RECORD], else AGR_EINVAL).  It takes
+ * ceil(len / 512) consecutive ring slots; AGR_EAGAIN when any of them still holds an uncollected answer.  agr_poll / agr_wait
+ * collect the ticket as usual.  agr_submit_ingest_var on a fixed-stride engine, and agr_submit_ingest on a variable-length one,
+ * return AGR_EINVAL. */
+int agr_submit_ingest_var(agr_handle* h, const uint8_t* rec, uint32_t len, agr_ticket* ticket);
 int agr_poll(agr_handle* h, agr_ticket ticket, agr_result* out);
 int agr_wait(agr_handle* h, agr_ticket ticket, agr_result* out);
 uint32_t agr_ring_capacity(void);
